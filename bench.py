@@ -3,10 +3,12 @@
 
 Workload (BASELINE.json configs[1]): Llama-3-8B, pure IQ4_NL (`llama-quantize --pure`), synthetic random-init weights.
 One "step" = one pass of the hot path over one batch:
-  * tg128: ONE token (n_batch = 1) through every MUL_MAT of the model, in graph order with real data dependencies:
+  * tg128: ONE token (n_batch = 1) through every MUL_MAT of the model, in graph order:
            32 x [ QKV (one multi-tensor mat-vec launch) -> wo -> fused up/gate/SiLU -> ffn_down ] -> output head.
            129 launches of our k_mmvq kernel and nothing else (attention/norm/rope are NOT the hot path and are not run;
-           the q projection is fed straight to wo so the chain keeps the dependency structure).
+           the q projection is fed straight to wo so the chain keeps the dependency structure).  On one GPU every layer's
+           Q,K,V read the same unit-rms activation in place of the RMS norm of the residual stream (see Model), so that
+           the logits are not zero.
   * pp512: the same matrices with n_batch = 512 through the tcgen05 GEMM path (head on the last token only,
            as llama-bench does); the SiLU*mul glue between up/gate and down is a torch elementwise op.
 Weights live in HBM in the plane layout (uploaded through the C-ABI repack); 4.2 GB of weights per pass >> 126 MB L2,
@@ -137,7 +139,10 @@ class Model:
         gen = torch.Generator(device="cuda")
         gen.manual_seed(seed + rank)
         # unit-gain weights (IQ4_NL codebook rms ~ 70).  There is no norm between the layers of this MUL_MAT-only skeleton and silu(g)*u makes the
-        # magnitude map quadratic, so the values contract towards 0 over the layers instead of overflowing the fp16 scale of q8_1
+        # magnitude map quadratic: chained from layer to layer the values would vanish within ~8 layers (all 32 then compute zeros) or
+        # overflow.  On one GPU the Q,K,V of every layer therefore read self.x, a unit-rms activation standing in for the normed residual
+        # stream; wo, up/gate and ffn_down still consume their predecessor's output, and the launches are the same.  The tensor-parallel
+        # paths keep the layer-to-layer chain: the fused kernels take the reduced output of the previous layer as their input
         s_e, s_f = 1.0 / (70.0 * N_EMBD ** 0.5), 1.0 / (70.0 * N_FF ** 0.5)
         # mix = "default": what `llama-quantize model IQ4_NL` produces WITHOUT --pure on this GQA model (src/llama-quantize.cpp:617-621, 739-745, 385-388):
         # attn_v -> IQ5_K, ffn_down of the first n_layer/8 layers -> Q5_K, output.weight -> Q6_K, everything else IQ4_NL
@@ -208,11 +213,12 @@ class Model:
         pf = getattr(be, "prefetch_next", lambda *a, **k: None)       # every launch warms the first stages of the NEXT launch's weights in L2
         nl = len(self.layers)
         for li, L in enumerate(self.layers):
+            xq = x if self.tp > 1 else self.x
             pf([L["wo"]])
             if L["wv"].ggml_type == L["wq"].ggml_type:
-                be.mul_mat_multi([L["wq"], L["wk"], L["wv"]], x, [self.q, self.kk, self.v])
+                be.mul_mat_multi([L["wq"], L["wk"], L["wv"]], xq, [self.q, self.kk, self.v])
             else:
-                be.mul_mat_multi([L["wq"], L["wk"]], x, [self.q, self.kk]); be.mul_mat(L["wv"], x, out=self.v)
+                be.mul_mat_multi([L["wq"], L["wk"]], xq, [self.q, self.kk]); be.mul_mat(L["wv"], xq, out=self.v)
             pf([L["up"]], gate=L["gate"])
             be.mul_mat(L["wo"], self.q, out=self.h); self.allreduce(self.h)
             pf([L["down"]])
@@ -232,12 +238,13 @@ class Model:
         x = self.x
         have_xb = False
         for li, L in enumerate(self.layers):
+            xq = x if self.tp > 1 else self.x
             if not have_xb:
-                be.convert_activations(x, self.xb)      # f32 -> bf16 once per distinct activation (shared by Q,K,V)
+                be.convert_activations(xq, self.xb)     # f32 -> bf16 once per distinct activation (shared by Q,K,V)
             if L["wv"].ggml_type == L["wq"].ggml_type:
-                be.mul_mat_multi([L["wq"], L["wk"], L["wv"]], x, [self.q, self.kk, self.v], x_bf16=self.xb)      # one launch
+                be.mul_mat_multi([L["wq"], L["wk"], L["wv"]], xq, [self.q, self.kk, self.v], x_bf16=self.xb)      # one launch
             else:
-                be.mul_mat_multi([L["wq"], L["wk"]], x, [self.q, self.kk], x_bf16=self.xb); be.mul_mat(L["wv"], x, out=self.v, x_bf16=self.xb)
+                be.mul_mat_multi([L["wq"], L["wk"]], xq, [self.q, self.kk], x_bf16=self.xb); be.mul_mat(L["wv"], xq, out=self.v, x_bf16=self.xb)
             be.convert_activations(self.q, self.qb)
             be.mul_mat(L["wo"], self.q, out=self.h, x_bf16=self.qb)
             if self.bf16_reduce:
@@ -261,7 +268,7 @@ class Model:
             be.mul_mat(self.head, x[-1:], out=self.logits)
 
 
-def bitnet_line(be, torch, steps, warmup, hbm_peak):
+def bitnet_line(be, torch, steps, warmup, hbm_peak, outputs):
     """BASELINE.json configs[3] / SURVEY App. A config 4: bitnet-b1.58-3B (n_embd 3200, n_ff 8640, 26 layers), IQ2_BN (2.0 bpw + f32 row scale), the
     per-layer MUL_MAT nodes only (the output matrix of that model is not IQ2_BN).  K = 3200 / 8640 are not multiples of 256: decode takes the TMA ring
     through the byte-granular geometry, prefill the int8 tensor-core path (ternary x int8 activations, tcgen05 kind::i8)."""
@@ -281,14 +288,13 @@ def bitnet_line(be, torch, steps, warmup, hbm_peak):
         x, q, k_, v, h, a, x2 = f(n, E), f(n, E), f(n, E), f(n, E), f(n, E), f(n, FF), f(n, E)
         x.normal_()
         def step():
-            cur = x
             for L in layers:
-                be.mul_mat_multi([L["wq"], L["wk"], L["wv"]], cur, [q, k_, v])
+                be.mul_mat_multi([L["wq"], L["wk"], L["wv"]], x, [q, k_, v])      # every layer reads the unit-rms x, as in Model
                 be.mul_mat(L["wo"], q, out=h)
                 be.fused_up_gate(L["up"], L["gate"], h, "silu", out=a)
                 be.mul_mat(L["down"], a, out=x2)
-                cur = x2
-        ms = time_graph(torch, step, steps if n == 1 else max(3, min(steps, 10)), warmup)
+        ms = time_graph(torch, step, steps, warmup)
+        outputs[f"bitnet_{'tg' if n == 1 else 'pp512'}_hidden"] = x2
         if n == 1:
             ach = wbytes / (ms * 1e-3) / 1e9
             out["tg"] = {"value": 1000.0 / ms, "unit": "tok/s", "ms_per_step": ms, "launches_per_step": 4 * NL,
@@ -431,7 +437,13 @@ def main():
     ap.add_argument("--no-pp", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-mix", action="store_true", help="skip the default-quantisation-mix line (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what each timed path computed in its last step "
+                    "(logits, final hidden states) as DIR/<name>.npy, float32; the inputs are seeded, so runs of two builds compare output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     config = {"reduce": "b200q NVLS kernel" if world > 1 and os.environ.get("B200Q_NCCL_REDUCE", "0") != "1" else ("nccl" if world > 1 else "none"), "workload": "Llama-3-8B pure IQ4_NL, llama-bench tg128 (n_batch=1) / pp512 (n_ubatch=512): all MUL_MAT nodes in graph order",
@@ -475,6 +487,12 @@ def main():
         os.environ.setdefault("NCCL_DEBUG", "WARN")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     torch.manual_seed(0)
+    # name -> host copy of what a timed path computed in its last step, taken right after that path's timing, before its buffers are reused
+    outputs = {}
+
+    def keep(**ts):
+        if args.dump_outputs:
+            outputs.update({k: t.float().cpu() for k, t in ts.items()})
 
     model = Model(be, torch, args.layers, tp=world, rank=rank)
     if model.fused_tp:
@@ -507,6 +525,7 @@ def main():
     with ClockSampler(local_rank) as cs:
         ms_tg = time_graph(torch, model.step_tg, args.steps, args.warmup, dist)
     clocks = cs.summary()
+    keep(tg_logits=model.logits)
     ms_tg_e2e = time_graph(torch, model.step_tg, args.steps, args.warmup, dist,
                            pre=lambda: model.x.copy_(x_host, non_blocking=True),
                            post=lambda: (logits_host.copy_(model.logits, non_blocking=True), torch.cuda.current_stream().synchronize()))
@@ -545,14 +564,14 @@ def main():
         model.alloc(n)
         xh = torch.randn(n, N_EMBD).pin_memory()
         model.x.copy_(xh)
-        pp_steps = max(3, min(args.steps, 10))
-        ms_pp = time_graph(torch, model.step_pp, pp_steps, args.warmup, dist)
-        ms_pp_e2e = time_graph(torch, model.step_pp, pp_steps, args.warmup, dist,
+        ms_pp = time_graph(torch, model.step_pp, args.steps, args.warmup, dist)
+        keep(pp512_logits=model.logits, pp512_hidden=model.x2)
+        ms_pp_e2e = time_graph(torch, model.step_pp, args.steps, args.warmup, dist,
                                pre=lambda: model.x.copy_(xh, non_blocking=True),
                                post=lambda: (logits_host.copy_(model.logits, non_blocking=True), torch.cuda.current_stream().synchronize()))
         fl = model_flops_pp(n, args.layers) / world
         tfs = fl / (ms_pp * 1e-3) / 1e12
-        line["pp512"] = {"metric": "llama-bench pp512 tok/s (MUL_MAT hot path)", "value": n * 1000.0 / ms_pp, "unit": "tok/s", "ms_per_step": ms_pp, "steps": pp_steps,
+        line["pp512"] = {"metric": "llama-bench pp512 tok/s (MUL_MAT hot path)", "value": n * 1000.0 / ms_pp, "unit": "tok/s", "ms_per_step": ms_pp, "steps": args.steps,
                          "dtype": "bf16 x bf16 -> f32 (tcgen05 kind::f16)", "e2e": {"value": n * 1000.0 / ms_pp_e2e, "unit": "tok/s", "h2d_bytes_per_step": n * N_EMBD * 4, "d2h_bytes_per_step": (N_VOCAB // world) * 4},
                          "roofline": {"bound": "tensor", "kernel": "k_gemm_q<IQ4_NL> (fused dequant + tcgen05; + k_f32_to_bf16)", "achieved": tfs, "peak": tf_peak, "unit": "TFLOP/s", "frac": tfs / tf_peak,
                                       "traffic": traffic.get("pp", {}).get("dram_bytes_per_step_gemm_only"), "traffic_source": traffic_src, "algorithmic_flops_per_step": fl,
@@ -564,13 +583,15 @@ def main():
         mm = Model(be, torch, args.layers, mix="default")
         mm.alloc(1); mm.x.copy_(x_host)
         ms_m = time_graph(torch, mm.step_tg, args.steps, args.warmup)
+        keep(mix_tg_logits=mm.logits)
         ach_m = mm.weight_bytes / (ms_m * 1e-3) / 1e9
         mix = {"workload": "same model, default `llama-quantize ... IQ4_NL` mix (no --pure): attn_v IQ5_K, ffn_down of layers 0-3 Q5_K, output.weight Q6_K",
                "tg": {"value": 1000.0 / ms_m, "unit": "tok/s", "ms_per_step": ms_m, "launches_per_step": mm.launches_tg,
                       "roofline": {"bound": "hbm", "achieved": ach_m, "peak": hbm_peak, "unit": "GB/s", "frac": ach_m / hbm_peak, "algorithmic_bytes_per_step": mm.weight_bytes}}}
         if not args.no_pp:
             mm.alloc(512); mm.x.copy_(xh)
-            ms_mp = time_graph(torch, mm.step_pp, pp_steps, args.warmup)
+            ms_mp = time_graph(torch, mm.step_pp, args.steps, args.warmup)
+            keep(mix_pp512_logits=mm.logits, mix_pp512_hidden=mm.x2)
             tfm = model_flops_pp(512, args.layers) / (ms_mp * 1e-3) / 1e12
             mix["pp512"] = {"value": 512 * 1000.0 / ms_mp, "unit": "tok/s", "ms_per_step": ms_mp,
                             "roofline": {"bound": "tensor", "achieved": tfm, "peak": tf_peak, "unit": "TFLOP/s", "frac": tfm / tf_peak}}
@@ -578,7 +599,9 @@ def main():
         del mm
         torch.cuda.empty_cache()
         try:
-            line["bitnet"] = bitnet_line(be, torch, args.steps, args.warmup, hbm_peak)
+            bitnet_out = {}
+            line["bitnet"] = bitnet_line(be, torch, args.steps, args.warmup, hbm_peak, bitnet_out)
+            keep(**bitnet_out)
         except Exception as e:      # a side line must never cost the headline
             line["bitnet"] = {"error": repr(e)}
     # ---------------- cpu baseline (rank 0, N=1 only) ----------------
@@ -593,6 +616,10 @@ def main():
                 line["cpu_baseline"] = cb
         except Exception as e:  # the baseline is a reported number, never a reason to lose the bench line
             line["cpu_baseline"] = {"error": repr(e)}
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in outputs.items():      # tensor parallel: each rank writes its own shard
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy" if world == 1 else f"{name}.rank{rank}.npy"), t.numpy())
     if rank == 0:
         print(json.dumps(line))
     if dist is not None:

@@ -92,8 +92,10 @@ def build_backend_ops_test(force: bool = False) -> str | None:
     if not os.path.exists(ref_lib):
         return None
     if force or _stale(exe, [src, plug]):
+        # libraries by file name (-L/-l), found through RUNPATH: full paths on the link line would be recorded as absolute DT_NEEDED
+        # entries, and the executable would not load once the tree is somewhere else
         subprocess.check_call(["g++", "-O2", "-std=c++17", "-o", exe, src, f"-I{REFERENCE_ROOT}/ggml/include", f"-I{REFERENCE_ROOT}/ggml/src",
-                               plug, ref_lib, os.path.join(HERE, "libb200q.so"), "-lpthread", "-ldl",
+                               f"-L{HERE}", "-lggml_b200", "-lb200q", f"-L{os.path.dirname(ref_lib)}", "-lggml_ref_avx2", "-lpthread", "-ldl",
                                "-Wl,-rpath,$ORIGIN/../../ik_llama_cpp_b200", "-Wl,-rpath,$ORIGIN/../../oracle/_ref"])
     return exe
 

@@ -6,7 +6,7 @@ from conftest import make_wire
 from ik_llama_cpp_b200 import backend as be
 from oracle.oracle import GGML_TYPE, Oracle
 orc = Oracle(); t = GGML_TYPE["IQ4_NL"]; n_expert, n_used, m, k, n_tokens = 5, 2, 132, 1024, 20
-wires = [make_wire(orc, "IQ4_NL", m, k, seed=900 + e) for e in range(n_expert)]
+wires = [make_wire("IQ4_NL", m, k, seed=900 + e) for e in range(n_expert)]
 W = be.set_expert_tensor(t, np.concatenate(wires), n_expert, m, k)
 rng = np.random.default_rng(3)
 for nb1 in (1, 2):

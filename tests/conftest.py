@@ -28,34 +28,18 @@ def oracle():
     return Oracle()
 
 
-@pytest.fixture(scope="session")
-def reflib():
-    """The unmodified reference CPU library, if oracle/_ref was built (needs /root/reference at build time)."""
-    from oracle.oracle import RefLib
-    if RefLib.find(prefer_native=False) is None:
-        pytest.skip("oracle/_ref not built")
-    return RefLib()
-
-
 def load_golden(name):
     z = np.load(os.path.join(GOLDEN_DIR, f"{name}.npz"))
     return {k: z[k] for k in z.files}
 
 
-def make_wire(oracle_or_ref, name, m, k, seed, reflib=None):
-    """Wire bytes for a random tensor.  With the reference library: real ggml_quantize_chunk output.
-    Without it (GPU box may lack it): random but VALID wire blocks (every bit pattern of the payload is a valid
-    encoding; scales are drawn as sane fp16/f32 values)."""
-    from oracle.oracle import GGML_TYPE
-    t = GGML_TYPE[name]
+def make_wire(name, m, k, seed, quantised=False):
+    """Wire bytes for a random tensor: random but VALID wire blocks (every bit pattern of the payload is a valid encoding; scales are
+    drawn as sane fp16/f32 values).  quantised=True, and always for the codebook / trellis / row-interleaved types: blocks and row
+    headers resampled from the golden tensor the reference's own quantiser produced, i.e. data with the statistics of real quantiser output."""
     rng = np.random.default_rng(seed)
-    if reflib is not None:
-        w = (rng.standard_normal((m, k)) * 0.02).astype(np.float32)
-        if name in ("IQ2_BN", "IQ1_BN"):
-            w = (rng.integers(-1, 2, (m, k)) * 0.043).astype(np.float32)
-        if name in _WIRE_GEOM and (m % _WIRE_GEOM[name][3] or name.endswith("_KT")):      # (the trellis quantisers take ~1 s per row: resample instead)
-            return random_wire(name, m, k, rng)
-        return reflib.quantize(t, w)
+    if quantised:
+        return _resample_golden_wire(name, m, k, rng)
     return random_wire(name, m, k, rng)
 
 
@@ -77,7 +61,7 @@ _WIRE_GEOM = {"IQ2_XXS": (256, 66, 0, 1), "IQ2_XS": (256, 74, 0, 1), "IQ3_XXS": 
 def _resample_golden_wire(name, m, k, rng):
     """Valid wire bytes of a wire-layout type without the reference library (GPU box): row groups assembled from randomly drawn blocks and
     row headers of the committed golden tensor (which the reference's own quantiser produced)."""
-    qk, bs, meta, il = _WIRE_GEOM[name]
+    qk, bs, meta, il = _WIRE_GEOM[name] if name in _WIRE_GEOM else (_QK.get(name, 256), _GEOM[name][0], _GEOM[name][2], 1)
     g = load_golden(name)
     gm, gk = int(g["m"]), int(g["k"])
     assert m % il == 0 and k % qk == 0

@@ -1,9 +1,14 @@
-"""The bench.py JSON contract, checked on the lines committed under profiles/ (produced on a B200 by scripts/gpu_profile_r1b.sh) and
-on the argument parser: a missing key would make the driver's BENCH_rNN.json unusable."""
+"""The bench.py JSON contract, checked on the lines committed under profiles/ (produced on a B200 by scripts/gpu_profile_r1b.sh), on
+the argument parser and (GPU) on a short run: a missing key would make the recorded bench results unusable."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
+
+from oracle.oracle import nmse
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = ["metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data", "config", "e2e"]
@@ -60,5 +65,28 @@ def test_traffic_file_matches_the_algorithmic_bytes():
 def test_bench_cli_defaults():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout, flag
+
+
+@pytest.mark.gpu
+def test_bench_steps_and_dump_outputs(tmp_path):
+    """--steps is the number of timed steps of every timed loop; --dump-outputs writes what the timed paths computed in their last step,
+    from inputs that are the same in every run.  All 32 layers: the outputs must not decay to zero on the way through the model."""
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--no-cpu", "--no-mix"]
+    dumps = []
+    for run in range(2):
+        out = tmp_path / str(run)
+        r = subprocess.run(cmd + ["--dump-outputs", str(out)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 2 and line["pp512"]["steps"] == 2 and line["gpu_launches"] == 2 * line["roofline"]["launches_per_step"]
+        dumps.append({f.stem: np.load(f) for f in out.glob("*.npy")})
+    assert sorted(dumps[0]) == ["pp512_hidden", "pp512_logits", "tg_logits"]
+    shapes = {"tg_logits": (1, 128256), "pp512_logits": (1, 128256), "pp512_hidden": (512, 4096)}
+    for name, a in dumps[0].items():
+        assert a.dtype == np.float32 and a.shape == shapes[name] and np.isfinite(a).all(), name
+        assert float(np.sqrt((a.astype(np.float64) ** 2).mean())) > 1e-2, (name, "outputs vanish")
+        # same inputs, so only the order of the split-K GEMM's f32 atomic adds may differ (other inputs would give an NMSE near 1)
+        e = nmse(dumps[1][name], a)
+        assert e <= 1e-4, (name, e)

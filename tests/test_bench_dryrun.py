@@ -64,3 +64,29 @@ def test_model_skeleton_walks_tg_and_pp(monkeypatch):
     assert be.calls.count("multi") == 2 and be.calls.count("mul_mat") == 7 and mm.launches_tg == 11
     assert mm.head.ggml_type == 14 and mm.layers[0]["down"].ggml_type == 13 and mm.layers[1]["wv"].ggml_type == 140
     mm.alloc(512); mm.step_pp()
+
+
+def test_time_graph_times_exactly_steps_replays():
+    """--steps is the timed loop count: time_graph brackets exactly `steps` graph replays with its two timing events and divides by steps."""
+    log = []
+
+    class _Ctx:
+        def __enter__(self): return self
+        def __exit__(self, *a): return False
+
+    class _Event:
+        def __init__(self, enable_timing=False): pass
+        def record(self): log.append("record")
+        def elapsed_time(self, other): return 14.0
+
+    class _Graph:
+        def replay(self): log.append("replay")
+
+    stream = types.SimpleNamespace(wait_stream=lambda s: None)
+    cuda = types.SimpleNamespace(Stream=lambda: stream, current_stream=lambda: stream, stream=lambda s: _Ctx(), synchronize=lambda: None,
+                                 CUDAGraph=_Graph, graph=lambda g: _Ctx(), Event=_Event)
+    for steps in (1, 7, 40):
+        log.clear()
+        ms = bench.time_graph(types.SimpleNamespace(cuda=cuda), lambda: log.append("eager"), steps, warmup=2)
+        i0, i1 = log.index("record"), len(log) - 1 - log[::-1].index("record")
+        assert log[i0 + 1:i1] == ["replay"] * steps and ms == 14.0 / steps

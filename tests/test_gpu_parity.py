@@ -29,12 +29,6 @@ def be():
     return backend
 
 
-@pytest.fixture(scope="module")
-def ref_or_none():
-    from oracle.oracle import RefLib
-    return RefLib() if RefLib.find(prefer_native=False) else None
-
-
 def rms(a):
     return float(np.sqrt((a.astype(np.float64) ** 2).mean()))
 
@@ -96,10 +90,10 @@ def test_golden_mat_vec(be, oracle, name):
 
 @pytest.mark.parametrize("name", ALL_TYPES)
 @pytest.mark.parametrize("n", [1, 2, 3, 5, 8])
-def test_mat_vec_vs_oracle(be, oracle, ref_or_none, name, n):
+def test_mat_vec_vs_oracle(be, oracle, name, n):
     t = GGML_TYPE[name]
     m, k = (260 if name.endswith("_R4") else 257), 2048      # ragged M (not a multiple of the CTA tile; the _R4 repacks come in groups of 4 rows)
-    wire = make_wire(oracle, name, m, k, seed=11 + t + n, reflib=ref_or_none)
+    wire = make_wire(name, m, k, seed=11 + t + n, quantised=True)
     rng = np.random.default_rng(5 + n)
     x = rng.standard_normal((n, k)).astype(np.float32)
     x[0, 64:96] = 0.0                      # amax == 0 block
@@ -119,7 +113,7 @@ def test_k_not_multiple_of_256(be, oracle, name, k, n):
     the TMA ring needs K % 256 == 0, these shapes take the LDG mat-vec / the zero-filled last GEMM k-block."""
     t = GGML_TYPE[name]
     m = 130
-    wire = make_wire(oracle, name, m, k, seed=300 + n)
+    wire = make_wire(name, m, k, seed=300 + n)
     x = np.random.default_rng(50 + n).standard_normal((n, k)).astype(np.float32)
     w = be.set_tensor(t, wire, m, k)
     assert np.array_equal(be.get_tensor(w), np.frombuffer(wire, np.uint8))
@@ -134,11 +128,11 @@ def test_k_not_multiple_of_256(be, oracle, name, k, n):
 
 
 @pytest.mark.parametrize("name", ["IQ4_NL", "Q4_K", "Q6_K", "IQ5_K"])
-def test_mat_vec_llama_shapes(be, oracle, ref_or_none, name):
+def test_mat_vec_llama_shapes(be, oracle, name):
     """BASELINE config 1: MUL_MAT 4096x4096 n=1 (and the 14336-wide FFN shape) at full size."""
     t = GGML_TYPE[name]
     for (m, k) in ((4096, 4096), (512, 14336)):
-        wire = make_wire(oracle, name, m, k, seed=3, reflib=None)
+        wire = make_wire(name, m, k, seed=3)
         x = np.random.default_rng(1).standard_normal((1, k)).astype(np.float32)
         w = be.set_tensor(t, wire, m, k)
         y = be.mul_mat(w, torch.from_numpy(x).cuda()).cpu().numpy()
@@ -153,10 +147,10 @@ def test_mat_vec_full_size_ffn_and_head_shapes(be, oracle, name):
     t = GGML_TYPE[name]
     x_rng = np.random.default_rng(21)
     for (m, k, glu) in ((14336, 4096, True), (32064, 4096, False), (4096, 14336, False)):
-        wire = make_wire(oracle, name, m, k, seed=5)
+        wire = make_wire(name, m, k, seed=5)
         w = be.set_tensor(t, wire, m, k)
         if glu:
-            wire2 = make_wire(oracle, name, m, k, seed=6); w2 = be.set_tensor(t, wire2, m, k)
+            wire2 = make_wire(name, m, k, seed=6); w2 = be.set_tensor(t, wire2, m, k)
         for it in range(3):
             x = x_rng.standard_normal((1, k)).astype(np.float32)
             xg = torch.from_numpy(x).cuda()
@@ -175,7 +169,7 @@ def test_multi_tensor_launch_qkv(be, oracle):
     t = GGML_TYPE["IQ4_NL"]
     k = 1024
     ms = [512, 128, 128]
-    wires = [make_wire(oracle, "IQ4_NL", m, k, seed=20 + i) for i, m in enumerate(ms)]
+    wires = [make_wire("IQ4_NL", m, k, seed=20 + i) for i, m in enumerate(ms)]
     ws = [be.set_tensor(t, wire, m, k) for wire, m in zip(wires, ms)]
     x = np.random.default_rng(2).standard_normal((2, k)).astype(np.float32)
     outs = be.mul_mat_multi(ws, torch.from_numpy(x).cuda())
@@ -191,7 +185,7 @@ def test_fused_up_gate(be, oracle, name, unary, limit, n):
     """n = 1, 2: the TMA-ring kernel; n = 5: the LDG kernel.  limit: after the activation, silu only (gelu ignores it)."""
     t = GGML_TYPE[name]
     m, k = 384, 1024
-    wu, wg = make_wire(oracle, name, m, k, seed=31), make_wire(oracle, name, m, k, seed=32)
+    wu, wg = make_wire(name, m, k, seed=31), make_wire(name, m, k, seed=32)
     x = np.random.default_rng(3).standard_normal((n, k)).astype(np.float32) * 4
     up, gate = be.set_tensor(t, wu, m, k), be.set_tensor(t, wg, m, k)
     y = be.fused_up_gate(up, gate, torch.from_numpy(x).cuda(), unary=unary, limit=limit).cpu().numpy()
@@ -200,18 +194,18 @@ def test_fused_up_gate(be, oracle, name, unary, limit, n):
     assert np.abs(y - ref).max() <= 5e-5 * max(rms(ref), 1e-30)
 
 
-def test_fused_up_gate_limit_matches_reference_cpu_op(be, oracle, ref_or_none):
-    """The clamp semantics pinned on the reference itself: GGML_OP_FUSED_UP_GATE with op_params limit through the unmodified CPU backend."""
-    if ref_or_none is None or not hasattr(ref_or_none.lib, "refshim_fused_up_gate"):
-        pytest.skip("reference CPU build (oracle/_ref) without the FUSED_UP_GATE shim")
+def test_fused_up_gate_limit_matches_reference_cpu_op(be, oracle):
+    """The clamp semantics pinned on the reference itself: GGML_OP_FUSED_UP_GATE with op_params limit through the unmodified CPU backend,
+    recorded in reference_xcheck.npz (tests/golden/gen_golden.py --xcheck)."""
+    g = load_golden("reference_xcheck")
     t = GGML_TYPE["Q4_0"]
     m, k = 256, 512
-    wu, wg = make_wire(oracle, "Q4_0", m, k, seed=61), make_wire(oracle, "Q4_0", m, k, seed=62)
+    wu, wg = make_wire("Q4_0", m, k, seed=61), make_wire("Q4_0", m, k, seed=62)
     x = np.random.default_rng(9).standard_normal((1, k)).astype(np.float32) * 6
     up, gate = be.set_tensor(t, wu, m, k), be.set_tensor(t, wg, m, k)
     for limit in (0.0, 1.5):
         y = be.fused_up_gate(up, gate, torch.from_numpy(x).cuda(), unary="silu", limit=limit).cpu().numpy()
-        r = ref_or_none.fused_up_gate(t, wu, wg, x, m, "silu", limit)
+        r = g[f"fused_up_gate.Q4_0.silu.limit{limit}"]
         assert nmse(y, r) <= 5e-4, (limit, nmse(y, r))
 
 
@@ -221,7 +215,7 @@ def test_q8_handoff_up_gate_to_down(be, oracle, name):
     Bit-identical to the path that re-quantises per CTA (same arithmetic on the same f32 values), and equal to the oracle."""
     t = GGML_TYPE[name]
     k, ff, m2 = (1024, 1536, 512) if name != "Q6_K" else (2048, 2048, 256)     # Q6_K's 2-byte d plane is bulk-copyable only for K % 2048 == 0
-    wu, wg, wd = make_wire(oracle, name, ff, k, seed=71), make_wire(oracle, name, ff, k, seed=72), make_wire(oracle, name, m2, ff, seed=73)
+    wu, wg, wd = make_wire(name, ff, k, seed=71), make_wire(name, ff, k, seed=72), make_wire(name, m2, ff, seed=73)
     up, gate, down = be.set_tensor(t, wu, ff, k), be.set_tensor(t, wg, ff, k), be.set_tensor(t, wd, m2, ff)
     x = torch.from_numpy(np.random.default_rng(4).standard_normal((1, k)).astype(np.float32) * 3).cuda()
     q8 = be.Q8Scratch(ff)
@@ -251,7 +245,7 @@ def test_mat_vec_bias(be, oracle, name, n):
     import ik_llama_cpp_b200 as pkg
     t = GGML_TYPE[name]
     m, k = 322, 1024
-    wire = make_wire(oracle, name, m, k, seed=81)
+    wire = make_wire(name, m, k, seed=81)
     w = be.set_tensor(t, wire, m, k)
     x = np.random.default_rng(12).standard_normal((n, k)).astype(np.float32)
     bias = np.random.default_rng(13).standard_normal(m).astype(np.float32)
@@ -270,9 +264,9 @@ def test_mul_mat_id(be, oracle, name, n_tokens, nb1, glu):
     Oracle: the plain mat-vec oracle on the selected expert's wire bytes."""
     t = GGML_TYPE[name]
     n_expert, n_used, m, k = 6, 3, 260, 1024
-    rs = len(make_wire(oracle, name, 4, k, seed=1)) // 4
-    wires = [make_wire(oracle, name, m, k, seed=400 + e) for e in range(n_expert)]
-    gwires = [make_wire(oracle, name, m, k, seed=500 + e) for e in range(n_expert)]
+    rs = len(make_wire(name, 4, k, seed=1)) // 4
+    wires = [make_wire(name, m, k, seed=400 + e) for e in range(n_expert)]
+    gwires = [make_wire(name, m, k, seed=500 + e) for e in range(n_expert)]
     assert all(len(w) == m * rs for w in wires)
     W = be.set_expert_tensor(t, np.concatenate(wires), n_expert, m, k)
     G = be.set_expert_tensor(t, np.concatenate(gwires), n_expert, m, k) if glu else None
@@ -317,10 +311,10 @@ def test_add_rows(be):
 
 @pytest.mark.parametrize("name", ALL_TYPES)
 @pytest.mark.parametrize("n", [16, 33, 512])
-def test_gemm_vs_oracle(be, oracle, ref_or_none, name, n):
+def test_gemm_vs_oracle(be, oracle, name, n):
     t = GGML_TYPE[name]
     m, k = (384, 1024) if n == 512 else (200, 512)        # ragged M and N
-    wire = make_wire(oracle, name, m, k, seed=41 + t, reflib=ref_or_none)
+    wire = make_wire(name, m, k, seed=41 + t, quantised=True)
     x = np.random.default_rng(6 + n).standard_normal((n, k)).astype(np.float32)
     w = be.set_tensor(t, wire, m, k)
     y = be.mul_mat(w, torch.from_numpy(x).cuda()).cpu().numpy()
@@ -340,7 +334,7 @@ def test_bitnet_int8_gemm_is_exact_integer_arithmetic(be, oracle, m, k, n):
     bitnet-b1.58 row lengths (not multiples of the 128-wide k-block: zero-filled TMA tails), K = 64 a single wire block."""
     import ik_llama_cpp_b200 as pkg
     t = GGML_TYPE["IQ2_BN"]
-    wire = make_wire(oracle, "IQ2_BN", m, k, seed=400 + n)
+    wire = make_wire("IQ2_BN", m, k, seed=400 + n)
     x = (np.random.default_rng(60 + n).standard_normal((n, k)) * 1.7).astype(np.float32)
     x[0, :] = 0.0                                           # an all-zero token (amax == 0)
     w = be.set_tensor(t, wire, m, k)
@@ -368,7 +362,7 @@ def test_gemm_shared_activation_and_unfused_path(be, oracle, name):
     import ik_llama_cpp_b200 as pkg
     t = GGML_TYPE[name]
     m, k, n = 256, 768, 40
-    wire = make_wire(oracle, name, m, k, seed=91 + t)
+    wire = make_wire(name, m, k, seed=91 + t)
     x = np.random.default_rng(17).standard_normal((n, k)).astype(np.float32)
     w = be.set_tensor(t, wire, m, k)
     xg = torch.from_numpy(x).cuda()
@@ -392,7 +386,7 @@ def test_gemm_multi_tensor_launch_qkv(be, oracle, name, n):
     t = GGML_TYPE[name]
     k = 1024
     ms = [512, 128, 200]
-    wires = [make_wire(oracle, name, m, k, seed=120 + i) for i, m in enumerate(ms)]
+    wires = [make_wire(name, m, k, seed=120 + i) for i, m in enumerate(ms)]
     ws = [be.set_tensor(t, wire, m, k) for wire, m in zip(wires, ms)]
     x = np.random.default_rng(21).standard_normal((n, k)).astype(np.float32)
     xg = torch.from_numpy(x).cuda()
@@ -415,7 +409,7 @@ def test_fused_up_gate_gemm(be, oracle, name, m, k, unary, limit, fuse):
     gate GEMM + k_mul_unary.  Checked against act(gate.x)*(up.x) from the plain GEMM entry point and the oracle."""
     t = GGML_TYPE[name]
     n = 70
-    wu, wg = make_wire(oracle, name, m, k, seed=131), make_wire(oracle, name, m, k, seed=132)
+    wu, wg = make_wire(name, m, k, seed=131), make_wire(name, m, k, seed=132)
     up, gate = be.set_tensor(t, wu, m, k), be.set_tensor(t, wg, m, k)
     x = np.random.default_rng(23).standard_normal((n, k)).astype(np.float32) * 2
     xg = torch.from_numpy(x).cuda()
@@ -449,7 +443,7 @@ def test_gemm_llama_shape_properties(be, oracle):
     t = GGML_TYPE["IQ4_NL"]
     m = k = 4096
     n = 512
-    wire = make_wire(oracle, "IQ4_NL", m, k, seed=77)
+    wire = make_wire("IQ4_NL", m, k, seed=77)
     x = np.random.default_rng(8).standard_normal((n, k)).astype(np.float32)
     w = be.set_tensor(t, wire, m, k)
     xg = torch.from_numpy(x).cuda()
@@ -466,7 +460,7 @@ def test_gemm_llama_shape_properties(be, oracle):
 def test_host_buffer_entry_point(be, oracle):
     t = GGML_TYPE["Q4_K"]
     m, k = 320, 1024
-    wire = make_wire(oracle, "Q4_K", m, k, seed=51)
+    wire = make_wire("Q4_K", m, k, seed=51)
     w = be.set_tensor(t, wire, m, k)
     for n in (1, 24):
         x = np.random.default_rng(n).standard_normal((n, k)).astype(np.float32)
