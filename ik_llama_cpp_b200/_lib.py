@@ -79,6 +79,11 @@ def lib() -> ctypes.CDLL:
     if hasattr(L, "b200q_mul_mat_id_vec"):
         L.b200q_mul_mat_id_vec.argtypes = [i32, vp, vp, i32, vp, vp, vp, i64, i64, i32, i32, i32, i32, c_float, vp]
         L.b200q_add_rows.argtypes = [vp, vp, vp, i64, i64, i64, vp]
+    if hasattr(L, "b200q_mul_mat_id_gemm"):
+        L.b200q_mul_mat_id_workspace.restype = c_size_t
+        L.b200q_mul_mat_id_workspace.argtypes = [i32, i64, i64, i32, i32, i32, i32, i32]
+        L.b200q_mul_mat_id_gemm.argtypes = [i32, vp, vp, i32, vp, vp, vp, i64, i64, i32, i32, i32, i32, c_float, vp, c_size_t, vp]
+        L.b200q_mul_mat_id.argtypes = [i32, vp, vp, i32, vp, vp, vp, i64, i64, i32, i32, i32, i32, c_float, vp, c_size_t, vp]
     if hasattr(L, "b200q_decode_prefetch_next"):
         L.b200q_decode_prefetch_next.argtypes = [i32, i32, vp, vp, vp, i64]
     _lib = L

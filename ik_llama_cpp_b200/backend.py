@@ -270,18 +270,52 @@ def set_expert_tensor(ggml_type: int, wire, n_expert: int, m: int, k: int, devic
     return ExpertTensor(ggml_type, n_expert, m, k, planes)
 
 
-def mul_mat_id(w: ExpertTensor, x: torch.Tensor, ids: torch.Tensor, gate: "ExpertTensor | None" = None, unary: str = "silu", limit: float = 0.0) -> torch.Tensor:
-    """GGML_OP_MUL_MAT_ID (gate is None) / GGML_OP_MOE_FUSED_UP_GATE for small batches: x f32 [n_tokens, nb1, K], ids int32 [n_tokens, n_used]
-    -> dst f32 [n_tokens, n_used, M] with dst[t, e] = W[ids[t, e]] . x[t, e % nb1]  (gate: unary(gate[id] . x) * (W[id] . x))."""
-    _require_cuda()
+def _check_mul_mat_id(w: ExpertTensor, x: torch.Tensor, ids: torch.Tensor, gate: "ExpertTensor | None"):
     assert x.is_cuda and x.dtype == torch.float32 and x.dim() == 3 and x.is_contiguous() and x.shape[2] == w.k
     assert ids.is_cuda and ids.dtype == torch.int32 and ids.dim() == 2 and ids.is_contiguous() and ids.shape[0] == x.shape[0]
+    assert gate is None or (gate.ggml_type == w.ggml_type and gate.n_expert == w.n_expert and gate.m == w.m and gate.k == w.k)
     n_tokens, nb1, n_used = x.shape[0], x.shape[1], ids.shape[1]
     assert n_used % nb1 == 0
+    return n_tokens, nb1, n_used
+
+
+def mul_mat_id(w: ExpertTensor, x: torch.Tensor, ids: torch.Tensor, gate: "ExpertTensor | None" = None, unary: str = "silu", limit: float = 0.0,
+               dispatch: bool = False) -> torch.Tensor:
+    """GGML_OP_MUL_MAT_ID (gate is None) / GGML_OP_MOE_FUSED_UP_GATE: x f32 [n_tokens, nb1, K], ids int32 [n_tokens, n_used]
+    -> dst f32 [n_tokens, n_used, M] with dst[t, e] = W[ids[t, e]] . x[t, e % nb1]  (gate: unary(gate[id] . x) * (W[id] . x)).
+    dispatch=False: the mat-vec kernel at every batch size (b200q_mul_mat_id_vec); dispatch=True: what the graph nodes run (b200q_mul_mat_id:
+    the grouped GEMM for large batches of the types it covers, the mat-vec kernel otherwise)."""
+    _require_cuda()
+    n_tokens, nb1, n_used = _check_mul_mat_id(w, x, ids, gate)
     dst = torch.empty((n_tokens, n_used, w.m), dtype=torch.float32, device=x.device)
+    L = _lib.lib()
     with torch.cuda.device(x.device):
-        check(_lib.lib().b200q_mul_mat_id_vec(w.ggml_type, w.ptr, gate.ptr if gate is not None else None, w.n_expert, ids.data_ptr(), x.data_ptr(), dst.data_ptr(),
-                                              w.m, w.k, n_used, nb1, n_tokens, UNARY[unary], float(limit), _stream()), "b200q_mul_mat_id_vec")
+        if dispatch:
+            need = L.b200q_mul_mat_id_workspace(w.ggml_type, w.m, w.k, w.n_expert, n_used, nb1, n_tokens, int(gate is not None))
+            ws = _workspace(need, x.device) if need else None
+            check(L.b200q_mul_mat_id(w.ggml_type, w.ptr, gate.ptr if gate is not None else None, w.n_expert, ids.data_ptr(), x.data_ptr(), dst.data_ptr(),
+                                     w.m, w.k, n_used, nb1, n_tokens, UNARY[unary], float(limit), ws.data_ptr() if ws is not None else None, need, _stream()),
+                  "b200q_mul_mat_id")
+        else:
+            check(L.b200q_mul_mat_id_vec(w.ggml_type, w.ptr, gate.ptr if gate is not None else None, w.n_expert, ids.data_ptr(), x.data_ptr(), dst.data_ptr(),
+                                         w.m, w.k, n_used, nb1, n_tokens, UNARY[unary], float(limit), _stream()), "b200q_mul_mat_id_vec")
+    return dst
+
+
+def mul_mat_id_gemm(w: ExpertTensor, x: torch.Tensor, ids: torch.Tensor, gate: "ExpertTensor | None" = None, unary: str = "silu", limit: float = 0.0,
+                    out: torch.Tensor | None = None) -> torch.Tensor:
+    """The same op as mul_mat_id through the grouped tcgen05 GEMM at any batch size (b200q_mul_mat_id_gemm): routing, gather and GEMM stay on
+    the device, so the call can be captured in a CUDA graph.  Raises for types / shapes the grouped path does not cover."""
+    _require_cuda()
+    n_tokens, nb1, n_used = _check_mul_mat_id(w, x, ids, gate)
+    dst = out if out is not None else torch.empty((n_tokens, n_used, w.m), dtype=torch.float32, device=x.device)
+    assert dst.dtype == torch.float32 and dst.is_contiguous() and dst.shape == (n_tokens, n_used, w.m)
+    L = _lib.lib()
+    with torch.cuda.device(x.device):
+        need = L.b200q_mul_mat_id_workspace(w.ggml_type, w.m, w.k, w.n_expert, n_used, nb1, n_tokens, int(gate is not None))
+        ws = _workspace(max(need, 1), x.device)
+        check(L.b200q_mul_mat_id_gemm(w.ggml_type, w.ptr, gate.ptr if gate is not None else None, w.n_expert, ids.data_ptr(), x.data_ptr(), dst.data_ptr(),
+                                      w.m, w.k, n_used, nb1, n_tokens, UNARY[unary], float(limit), ws.data_ptr(), ws.numel(), _stream()), "b200q_mul_mat_id_gemm")
     return dst
 
 

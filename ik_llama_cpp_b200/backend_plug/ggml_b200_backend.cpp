@@ -251,7 +251,7 @@ GGML_CALL static bool b200_backend_supports_op(ggml_backend_t, const ggml_tensor
                    ggml_is_contiguous(op) && ggml_is_contiguous(op->src[0]) && ggml_is_contiguous(op->src[1]) && ggml_are_same_shape(op, op->src[0]) &&
                    op->src[1]->ne[0] == op->ne[0] && (ggml_nelements(op->src[1]) == op->ne[0] || ggml_are_same_shape(op, op->src[1]));
         case GGML_OP_MUL_MAT_ID: case GGML_OP_MOE_FUSED_UP_GATE: {
-            // MoE: expert ids resolved on the device; batches beyond the shared-memory capacity of one launch are walked in token chunks by the C ABI
+            // MoE: expert ids resolved on the device; large batches of the types the grouped GEMM covers take it, others are walked in token chunks by the mat-vec kernel
             const bool ug = op->op == GGML_OP_MOE_FUSED_UP_GATE;
             const ggml_tensor * w = op->src[0]; const ggml_tensor * g = ug ? op->src[1] : nullptr; const ggml_tensor * x = op->src[ug ? 2 : 1]; const ggml_tensor * ids = op->src[ug ? 3 : 2];
             if (!w || !x || !ids || (ug && (!g || g->type != w->type || !ggml_are_same_shape(g, w) || op->src[4] || op->src[5] || b200_unary(b200_op_param_i32(op, 0)) < 0))) return false;
@@ -337,8 +337,12 @@ GGML_CALL static enum ggml_status b200_backend_graph_compute(ggml_backend_t b, g
                 const bool ug = node->op == GGML_OP_MOE_FUSED_UP_GATE;
                 const ggml_tensor * w = node->src[0]; const ggml_tensor * g = ug ? node->src[1] : nullptr; const ggml_tensor * x = node->src[ug ? 2 : 1]; const ggml_tensor * ids = node->src[ug ? 3 : 2];
                 float limit = 0.0f; if (ug) memcpy(&limit, (const char *)node->op_params + sizeof(int32_t), sizeof(float));
-                B200Q_CHECK(b200q_mul_mat_id_vec(w->type, w->data, g ? g->data : nullptr, (int)w->ne[2], (const int32_t *)ids->data, (const float *)x->data, (float *)node->data,
-                                                 w->ne[1], w->ne[0], (int)ids->ne[0], (int)x->ne[1], (int)x->ne[2], ug ? b200_unary(b200_op_param_i32(node, 0)) : 0, limit, c->stream));
+                // decode-sized batches: the mat-vec kernel; larger batches of the covered types: the grouped GEMM (b200q_mul_mat_id dispatches)
+                const int n_expert = (int)w->ne[2], n_used = (int)ids->ne[0], nb1 = (int)x->ne[1], n_tokens = (int)x->ne[2];
+                const size_t need = b200q_mul_mat_id_workspace(w->type, w->ne[1], w->ne[0], n_expert, n_used, nb1, n_tokens, ug);
+                void * ws = need ? c->workspace(need) : nullptr;
+                B200Q_CHECK(b200q_mul_mat_id(w->type, w->data, g ? g->data : nullptr, n_expert, (const int32_t *)ids->data, (const float *)x->data, (float *)node->data,
+                                             w->ne[1], w->ne[0], n_used, nb1, n_tokens, ug ? b200_unary(b200_op_param_i32(node, 0)) : 0, limit, ws, need, c->stream));
             } break;
             case GGML_OP_FUSED_UP_GATE: {
                 const ggml_tensor * up = node->src[0]; const ggml_tensor * gate = node->src[1]; const ggml_tensor * x = node->src[2];

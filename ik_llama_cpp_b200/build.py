@@ -10,8 +10,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libb200q.so")
 OBJDIR = os.path.join(HERE, "_obj")
-SOURCES = ["b200q_decode_i0.cu", "b200q_decode_i1.cu", "b200q_decode_i2.cu", "b200q_decode_i3.cu", "b200q_wire.cu", "b200q_decode.cu", "b200q_gemm.cu", "b200q_reduce.cu", "b200q_api.cu"]
-HEADERS = ["b200q_types.cuh", "b200q_internal.h", "b200q_wire.cuh", "b200q_codebooks.h", "b200q_decode_common.cuh", "b200q_decode_ring.cuh", "b200q_decode_inst.inc", os.path.join("..", "..", "include", "b200q.h")]
+SOURCES = ["b200q_decode_i0.cu", "b200q_decode_i1.cu", "b200q_decode_i2.cu", "b200q_decode_i3.cu", "b200q_wire.cu", "b200q_decode.cu", "b200q_gemm.cu", "b200q_moe.cu", "b200q_reduce.cu", "b200q_api.cu"]
+HEADERS = ["b200q_types.cuh", "b200q_internal.h", "b200q_moe.cuh", "b200q_wire.cuh", "b200q_codebooks.h", "b200q_decode_common.cuh", "b200q_decode_ring.cuh", "b200q_decode_inst.inc", os.path.join("..", "..", "include", "b200q.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
 
@@ -78,26 +78,32 @@ def build_backend_plug(force: bool = False, verbose: bool = False) -> str | None
     return PLUG_LIB
 
 
+# harnesses under tests/backend_ops: test-backend-ops semantics through the real ggml-backend API (plug vs reference CPU backend)
+BACKEND_OPS_HARNESSES = ["test_mul_mat_backend", "test_moe_prefill_backend"]
+
+
 def build_backend_ops_test(force: bool = False) -> str | None:
-    """tests/backend_ops/test_mul_mat_backend: test-backend-ops semantics through the real ggml-backend API."""
+    """tests/backend_ops/test_mul_mat_backend (returned) and the other harnesses of BACKEND_OPS_HARNESSES, e.g. test_moe_prefill_backend
+    (MoE prefill through the plug's dispatcher)."""
     root = os.path.dirname(HERE)
-    exe = os.path.join(root, "tests", "backend_ops", "test_mul_mat_backend")
-    src = exe + ".cpp"
+    exes = [os.path.join(root, "tests", "backend_ops", name) for name in BACKEND_OPS_HARNESSES]
     if not os.path.isdir(REFERENCE_ROOT):
-        return exe if os.path.exists(exe) else None
+        return exes[0] if os.path.exists(exes[0]) else None
     plug = build_backend_plug(force)
     ref_lib = os.path.join(root, "oracle", "_ref", "libggml_ref_avx2.so")
     if plug is None:
         return None
     if not os.path.exists(ref_lib):
         return None
-    if force or _stale(exe, [src, plug]):
-        # libraries by file name (-L/-l), found through RUNPATH: full paths on the link line would be recorded as absolute DT_NEEDED
-        # entries, and the executable would not load once the tree is somewhere else
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-o", exe, src, f"-I{REFERENCE_ROOT}/ggml/include", f"-I{REFERENCE_ROOT}/ggml/src",
-                               f"-L{HERE}", "-lggml_b200", "-lb200q", f"-L{os.path.dirname(ref_lib)}", "-lggml_ref_avx2", "-lpthread", "-ldl",
-                               "-Wl,-rpath,$ORIGIN/../../ik_llama_cpp_b200", "-Wl,-rpath,$ORIGIN/../../oracle/_ref"])
-    return exe
+    for exe in exes:
+        src = exe + ".cpp"
+        if force or _stale(exe, [src, plug]):
+            # libraries by file name (-L/-l), found through RUNPATH: full paths on the link line would be recorded as absolute DT_NEEDED
+            # entries, and the executable would not load once the tree is somewhere else
+            subprocess.check_call(["g++", "-O2", "-std=c++17", "-o", exe, src, f"-I{REFERENCE_ROOT}/ggml/include", f"-I{REFERENCE_ROOT}/ggml/src",
+                                   f"-L{HERE}", "-lggml_b200", "-lb200q", f"-L{os.path.dirname(ref_lib)}", "-lggml_ref_avx2", "-lpthread", "-ldl",
+                                   "-Wl,-rpath,$ORIGIN/../../ik_llama_cpp_b200", "-Wl,-rpath,$ORIGIN/../../oracle/_ref"])
+    return exes[0]
 
 
 if __name__ == "__main__":

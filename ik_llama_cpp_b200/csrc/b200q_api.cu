@@ -403,7 +403,7 @@ int b200q_mul_mat_id_vec(int type, const void * W, const void * W_gate, int n_ex
     if (((uintptr_t)x & 15) || (k & 3)) return fail(B200Q_E_ARG, "b200q_mul_mat_id_vec: activations must be 16-byte aligned");
     if (n_tokens < 1 || n_used < 1 || nb1 < 1 || n_used % nb1) return fail(B200Q_E_ARG, "b200q_mul_mat_id_vec: bad token / slot counts");
     // the quantised activation columns of a launch live in shared memory: larger batches are walked in token chunks (same kernel, the expert ids
-    // never leave the device).  This is the functional path for MoE prefill, not a tuned one: a grouped tensor-core GEMM is not built.
+    // never leave the device).  b200q_mul_mat_id sends larger batches of the types the grouped tcgen05 GEMM covers there instead.
     const int64_t col_bytes = (int64_t)nb1 * (k + k / 4);
     int chunk = (int)((200 * 1024) / (col_bytes > 0 ? col_bytes : 1));
     static const int forced = [] { const char * e = getenv("B200Q_MOE_CHUNK_TOKENS"); return e ? atoi(e) : 0; }();
@@ -419,6 +419,40 @@ int b200q_mul_mat_id_vec(int type, const void * W, const void * W_gate, int n_ex
         if (rc) return rc;
     }
     return B200Q_OK;
+}
+size_t b200q_mul_mat_id_workspace(int type, int64_t m, int64_t k, int n_expert, int n_used, int nb1, int n_tokens, int up_gate) {
+    b200q_moe_plan_t p;
+    return b200q_moe_plan(type, m, k, n_expert, n_used, nb1, n_tokens, up_gate, &p) == 0 ? p.total : 0;
+}
+int b200q_mul_mat_id_gemm(int type, const void * W, const void * W_gate, int n_expert, const int32_t * ids, const float * x, float * dst,
+                          int64_t m, int64_t k, int n_used, int nb1, int n_tokens, int unary, float limit, void * workspace, size_t workspace_bytes, void * stream) {
+    if (!W || !ids || !x || !dst || !workspace || m <= 0 || k <= 0 || n_expert < 1) return fail(B200Q_E_ARG, "b200q_mul_mat_id_gemm: bad argument");
+    if (n_tokens < 1 || n_used < 1 || nb1 < 1 || n_used % nb1) return fail(B200Q_E_ARG, "b200q_mul_mat_id_gemm: bad token / slot counts");
+    if (((uintptr_t)x & 15) || ((uintptr_t)workspace & 255)) return fail(B200Q_E_ARG, "b200q_mul_mat_id_gemm: x must be 16-byte and the workspace 256-byte aligned");
+    b200q_moe_plan_t p;
+    const int rc = b200q_moe_plan(type, m, k, n_expert, n_used, nb1, n_tokens, W_gate != nullptr, &p);
+    if (rc == -1) return fail(B200Q_E_TYPE, "b200q_mul_mat_id_gemm: type %d has no grouped GEMM", type);
+    if (rc) return fail(B200Q_E_SHAPE, "b200q_mul_mat_id_gemm: shape not covered by the grouped GEMM (k %% 256 == 0, n_expert <= 512)");
+    if (workspace_bytes < p.total) return fail(B200Q_E_ARG, "b200q_mul_mat_id_gemm: workspace too small (%zu < %zu)", workspace_bytes, p.total);
+    dev_info & di = device_info(); if (!di.ok) return fail(B200Q_E_CUDA, "b200q_mul_mat_id_gemm: no CUDA device");
+    b200q_moe_desc d; memset(&d, 0, sizeof d);
+    d.type = type; d.W = W; d.W_gate = W_gate; d.n_expert = n_expert; d.ids = ids; d.x = x; d.dst = dst; d.M = m; d.K = k;
+    d.n_used = n_used; d.nb1 = nb1; d.n_tokens = n_tokens; d.act = unary; d.limit = limit;
+    return check_launch(b200q_launch_moe_gemm(d, p, workspace, (cudaStream_t)stream), "b200q_mul_mat_id_gemm");
+}
+// Smallest batch (routed rows n_tokens * n_used) that takes the grouped GEMM.  Measured with scripts/moe_prefill_bench.py on a B200 at a
+// 1000 W power limit (profiles/moe_prefill_b200.json, one MoE FFN layer, grouped GEMM vs mat-vec time): at 8 tokens the mat-vec kernel is
+// about as fast or faster (Qwen3-30B-A3B shape, 64 rows: IQ4_NL 1.05-1.15x, Q4_K 0.84-0.92x; Mixtral-8x7B shape, 16 rows: 1.03-1.10x /
+// 0.83-0.89x), at 16 tokens the grouped GEMM wins at every point (1.25-1.74x).  The crossover lies between 64 and 128 rows with 128
+// experts and between 16 and 32 rows with 8 experts: max(32, n_expert) rows puts both shapes on the measured winning side.
+static int64_t moe_gemm_min_rows(int n_expert) { return n_expert > 32 ? n_expert : 32; }
+int b200q_mul_mat_id(int type, const void * W, const void * W_gate, int n_expert, const int32_t * ids, const float * x, float * dst,
+                     int64_t m, int64_t k, int n_used, int nb1, int n_tokens, int unary, float limit, void * workspace, size_t workspace_bytes, void * stream) {
+    b200q_moe_plan_t p;
+    if (n_expert >= 1 && (int64_t)n_tokens * n_used >= moe_gemm_min_rows(n_expert) &&
+        b200q_moe_plan(type, m, k, n_expert, n_used, nb1, n_tokens, W_gate != nullptr, &p) == 0)
+        return b200q_mul_mat_id_gemm(type, W, W_gate, n_expert, ids, x, dst, m, k, n_used, nb1, n_tokens, unary, limit, workspace, workspace_bytes, stream);
+    return b200q_mul_mat_id_vec(type, W, W_gate, n_expert, ids, x, dst, m, k, n_used, nb1, n_tokens, unary, limit, stream);
 }
 int b200q_mul_mat_host(int type, const void * W, const float * x_host, float * dst_host, int64_t m, int64_t k, int64_t n, void * stream) {
     cudaStream_t st = (cudaStream_t)stream; cudaError_t e; int rc;

@@ -14,6 +14,7 @@
 //               coalesced f32 stores (the 32 lanes of a warp hold 32 consecutive m of the same token)
 // A comes either from the bf16 scratch written by k_dequant_bf16 (generic types) or ... (fused dequant: see k_gemm_q).
 #include "b200q_internal.h"
+#include "b200q_moe.cuh"
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -21,6 +22,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <type_traits>
 #include <unordered_map>
 
 namespace {
@@ -54,6 +56,11 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 __device__ __forceinline__ void tma_load_2d(void * smem_dst, const CUtensorMap * tm, uint64_t * bar, int x, int y) {
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                  ::"r"(smem_u32(smem_dst)), "l"((uint64_t)tm), "r"(smem_u32(bar)), "r"(x), "r"(y) : "memory");
+}
+// 3-D map {bytes along the row, row, expert}: the expert matrices of a MUL_MAT_ID weight tensor
+__device__ __forceinline__ void tma_load_3d(void * smem_dst, const CUtensorMap * tm, uint64_t * bar, int x, int y, int z) {
+    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+                 ::"r"(smem_u32(smem_dst)), "l"((uint64_t)tm), "r"(smem_u32(bar)), "r"(x), "r"(y), "r"(z) : "memory");
 }
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap * tm) {
     asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)tm) : "memory");
@@ -257,6 +264,12 @@ struct gemmq_args {
     gemmq_seg seg[GEMMQ_MAX_SEGS];
     int n_seg, N, K, k_split, act; float limit;
 };
+// grouped mode (MoE prefill, b200q_moe.cu): tmP* are 3-D maps {row bytes, M, n_expert}, tmB covers the expert-sorted bf16 activations
+// [n_rows][K]; blockIdx.y indexes the tile table, tiles at or beyond *n_tiles exit at once; column c of a tile is stored at output row
+// row_dst[col0 + c] of seg.dst.  Always k_split == 1: no memset, no atomics, every output is written exactly once.
+struct gemmq_gargs : gemmq_args {
+    const b200q_moe_tile * tiles; const int * n_tiles; const int * row_dst;
+};
 
 // carry-less per-byte add of two packed int8x4 (the A/B halves of the sign-fill LUT)
 __device__ __forceinline__ uint32_t vadd4_wrap(uint32_t a, uint32_t b) {
@@ -280,10 +293,17 @@ template <int J> __device__ __forceinline__ float biased_byte_to_float(uint32_t 
 // Pipelines: raw_full/raw_empty (TMA <-> dequant), a_full/a_empty (dequant <-> MMA), b_full/b_empty (TMA <-> MMA),
 // tmem_full (MMA -> epilogue).  Generic-proxy smem writes of the dequant warps are published to the tensor core with
 // fence.proxy.async before the a_full arrive.
-template <int TYPE, int NB>
+template <int TYPE, int NB, bool GROUPED = false>
 __global__ void __launch_bounds__(64 + 32 * DQ_WARPS, 1)
-k_gemm_q(const __grid_constant__ gemmq_args a) {
+k_gemm_q(const __grid_constant__ std::conditional_t<GROUPED, gemmq_gargs, gemmq_args> a) {
     using cfg = gemmq_cfg<TYPE, NB>;
+    int ex = 0, n_cols = 0;                                     // grouped: expert and valid columns of this tile
+    int n0 = blockIdx.y * cfg::BN;
+    if constexpr (GROUPED) {
+        if ((int)blockIdx.y >= __ldg(a.n_tiles)) return;        // beyond the routed tiles: leave before any barrier or TMEM allocation
+        const int4 tl = __ldg(reinterpret_cast<const int4 *>(a.tiles) + blockIdx.y);
+        ex = tl.x; n0 = tl.y; n_cols = tl.z - tl.y;
+    }
     int sg = 0;
 #pragma unroll
     for (int s = 1; s < GEMMQ_MAX_SEGS; ++s) if (s < a.n_seg && (int)blockIdx.x >= a.seg[s].tile0) sg = s;
@@ -304,7 +324,7 @@ k_gemm_q(const __grid_constant__ gemmq_args a) {
     uint32_t * tmem_slot = reinterpret_cast<uint32_t *>(tmem_full + 1);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int m0 = ((int)blockIdx.x - a.seg[sg].tile0) * BM, n0 = blockIdx.y * BN;
+    const int m0 = ((int)blockIdx.x - a.seg[sg].tile0) * BM;
     // K is walked in raw blocks of 256 weights; split-K over blockIdx.z in units of raw blocks
     const int nr_total = (K + RAW_K - 1) / RAW_K;
     const int nr_per = (nr_total + k_split - 1) / k_split;
@@ -336,9 +356,15 @@ k_gemm_q(const __grid_constant__ gemmq_args a) {
                 mbar_wait(&raw_empty[rs], rph ^ 1);
                 unsigned char * raw = sR + (size_t)rs * cfg::RAW_BYTES;
                 mbar_expect_tx(&raw_full[rs], cfg::RAW_BYTES);
+                if constexpr (GROUPED) {
+                    tma_load_3d(raw, tmP0, &raw_full[rs], (rb0 + r) * 128, m0, ex);
+                    tma_load_3d(raw + cfg::RAW_P0, tmP1, &raw_full[rs], (rb0 + r) * cfg::P1, m0, ex);
+                    if (cfg::P2) tma_load_3d(raw + cfg::RAW_P0 + cfg::RAW_P1, tmP2, &raw_full[rs], (rb0 + r) * cfg::P2, m0, ex);
+                } else {
                 tma_load_2d(raw, tmP0, &raw_full[rs], (rb0 + r) * 128, m0);                // bytes along the row
                 tma_load_2d(raw + cfg::RAW_P0, tmP1, &raw_full[rs], (rb0 + r) * cfg::P1, m0);
                 if (cfg::P2) tma_load_2d(raw + cfg::RAW_P0 + cfg::RAW_P1, tmP2, &raw_full[rs], (rb0 + r) * cfg::P2, m0);
+                }
                 for (int q = 0; q < RAW_K / BK && ib < nk; ++q, ++ib) {
                     const int s = ib % cfg::B_STAGES; const uint32_t ph = (ib / cfg::B_STAGES) & 1;
                     mbar_wait(&b_empty[s], ph ^ 1);
@@ -418,6 +444,30 @@ k_gemm_q(const __grid_constant__ gemmq_args a) {
             if (lane == 0) mbar_arrive(&raw_empty[rs]);
         }
         // ---------------- epilogue: quadrant q4, column half `half` ----------------
+        if constexpr (GROUPED) {
+            // columns past n_cols belong to the next expert or lie beyond n_rows: masked.  Lane j fetches the output row of column
+            // c0 + j once; the warp's 32 lanes (consecutive m) then store each column coalesced along M.
+            if (nk > 0) {
+                mbar_wait(tmem_full, 0);
+                tc_fence_after();
+                const int m = m0 + row;
+                constexpr int COLS_PER = BN / 2;
+                const int c_begin = half * COLS_PER, c_end = min((half + 1) * COLS_PER, n_cols);
+                const bool mrow = m < M;
+#pragma unroll 1
+                for (int c0 = c_begin; c0 < c_end; c0 += 32) {
+                    uint32_t rr[32];
+                    tmem_ld_32x32b_x32(tmem_base + ((uint32_t)(32 * q4) << 16) + (uint32_t)c0, rr);
+                    const int rd = c0 + lane < c_end ? __ldg(a.row_dst + n0 + c0 + lane) : 0;
+                    tmem_ld_wait();
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) {
+                        const int r = __shfl_sync(0xffffffffu, rd, j);
+                        if (mrow && c0 + j < c_end) dst[(size_t)r * M + m] = __uint_as_float(rr[j]);
+                    }
+                }
+            }
+        } else
         if (nk > 0) {
             mbar_wait(tmem_full, 0);
             tc_fence_after();
@@ -834,6 +884,47 @@ int launch_gemm_q(const b200q_gemm_multi & d, int k_split, cudaStream_t st) {
     return (int)cudaGetLastError();
 }
 
+// n_mat uint8 matrices [rows][row_bytes], mat_stride bytes apart: box = box_bytes x box_rows x 1 (one matrix per load)
+int make_tmap_u8_3d(CUtensorMap * tm, const void * ptr, int64_t n_mat, int64_t mat_stride, int64_t rows, int64_t row_bytes, int box_bytes, int box_rows, bool swizzle128) {
+    encode_tiled_fn enc = get_encode(); if (!enc) return -1;
+    cuuint64_t dims[3] = {(cuuint64_t)row_bytes, (cuuint64_t)rows, (cuuint64_t)n_mat};
+    cuuint64_t strides[2] = {(cuuint64_t)row_bytes, (cuuint64_t)mat_stride};
+    cuuint32_t box[3] = {(cuuint32_t)box_bytes, (cuuint32_t)box_rows, 1};
+    cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void *>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                     swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    return r == CUDA_SUCCESS ? 0 : -2;
+}
+
+// grouped (MoE) launch: ONE 3-D map per weight plane and segment, whatever n_expert; the grid covers the host-known bound on the tiles
+template <int TYPE, int NB>
+int launch_gemm_q_grouped(const b200q_gemm_grouped & g, cudaStream_t st) {
+    using cfg = gemmq_cfg<TYPE, NB>;
+    gemmq_gargs a; memset(&a, 0, sizeof a);
+    b200q_layout L; if (b200q_make_layout(TYPE, g.M, g.K, &L)) return -1;
+    const int64_t p1_row = (g.K / 256) * cfg::P1, p2_row = (g.K / 256) * cfg::P2;
+    int tiles = 0;
+    for (int i = 0; i < g.n_seg; ++i) {
+        const char * W = (const char *)g.W[i];
+        if (make_tmap_u8_3d(&a.tmP0[i], W + L.plane_off[0], g.n_expert, g.estride, g.M, g.K / 2, 128, BM, true)) return -10;
+        if (make_tmap_u8_3d(&a.tmP1[i], W + L.plane_off[1], g.n_expert, g.estride, g.M, p1_row, cfg::P1, BM, false)) return -13;
+        if (cfg::P2 && make_tmap_u8_3d(&a.tmP2[i], W + L.plane_off[2], g.n_expert, g.estride, g.M, p2_row, cfg::P2, BM, false)) return -13;
+        a.seg[i].dst = g.dst[i]; a.seg[i].M = (int)g.M; a.seg[i].tile0 = tiles;
+        tiles += (int)((g.M + BM - 1) / BM);
+    }
+    if (make_tmap_bf16(&a.tmB, g.xb, g.n_rows, g.K, NB == 0 ? 128 : 256)) return -11;
+    a.n_seg = g.n_seg; a.N = (int)g.n_rows; a.K = (int)g.K; a.k_split = 1;
+    a.tiles = (const b200q_moe_tile *)g.tiles; a.n_tiles = g.n_tiles; a.row_dst = g.row_dst;
+    static bool configured[B200Q_MAX_DEVICES] = {};
+    const int dev = b200q_current_device();
+    if (!configured[dev]) {
+        if (cudaFuncSetAttribute(k_gemm_q<TYPE, NB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg::SMEM) != cudaSuccess) return -12;
+        configured[dev] = true;
+    }
+    dim3 grid((unsigned)tiles, (unsigned)g.max_tiles, 1);
+    k_gemm_q<TYPE, NB, true><<<grid, 64 + 32 * DQ_WARPS, cfg::SMEM, st>>>(a);
+    return (int)cudaGetLastError();
+}
 
 // int8 activation tensor map: [rows][K bytes], box 128 bytes x box_rows, 128B swizzle, zero fill beyond K
 static int make_tmap_i8(CUtensorMap * tm, const void * ptr, int64_t rows, int64_t K, int box_rows) { return make_tmap_u8(tm, ptr, rows, K, 128, box_rows, true); }
@@ -881,6 +972,19 @@ int gemmq_choose_split(int64_t tiles, int64_t nr, int sm_count, bool allow_split
 
 }  // namespace
 
+
+int b200q_gemmq_type(int type) { return gemmq_supported(type) ? 1 : 0; }
+
+int b200q_launch_gemm_q_grouped(const b200q_gemm_grouped & g, cudaStream_t st) {
+    if (g.n_seg < 1 || g.n_seg > 2 || g.K % 256 || g.nb < 0 || g.nb > 2 || g.max_tiles < 1) return -2;
+    switch (g.type) {
+#define GQ(T) case T: return g.nb == 2 ? launch_gemm_q_grouped<T, 2>(g, st) : g.nb == 1 ? launch_gemm_q_grouped<T, 1>(g, st) : launch_gemm_q_grouped<T, 0>(g, st);
+        GQ(B200Q_TYPE_IQ4_NL) GQ(B200Q_TYPE_Q4_0) GQ(B200Q_TYPE_Q4_K) GQ(B200Q_TYPE_IQ4_K)
+        GQ(B200Q_TYPE_Q4_1) GQ(B200Q_TYPE_Q5_0) GQ(B200Q_TYPE_Q5_1) GQ(B200Q_TYPE_Q5_K) GQ(B200Q_TYPE_IQ5_K)
+#undef GQ
+        default: return -1;
+    }
+}
 
 // IQ2_BN prefill on the int8 tensor pipe.  X f32 [N][K] is quantised per token into `ws` (int8 [N][K] | ts[N] | sx[N]); up to 3 tensors share it.
 // Requires K % 64 == 0 (16-byte TMA strides); returns -100 when the shape is not eligible (callers use the bf16 path).

@@ -100,3 +100,24 @@ size_t b200q_gemm_i8_workspace_bytes(int64_t K, int64_t N);
 int b200q_launch_gemm_bn_i8(const b200q_gemm_multi & d, const float * x, int64_t x_stride, void * ws, size_t ws_bytes, cudaStream_t st);
 int b200q_launch_add_rows(const float * a, const float * b, float * dst, int64_t m, int64_t n, int64_t nb, cudaStream_t st);
 int b200q_launch_f32_to_bf16(const float * x, int64_t x_stride, void * out, int64_t K, int64_t N, cudaStream_t st);
+
+// MoE prefill (b200q_moe.cu): grouped k_gemm_q over expert-sorted token tiles
+int b200q_gemmq_type(int type);          // 1 if k_gemm_q decodes this type inside the kernel
+struct b200q_gemm_grouped {
+    int type; int n_seg; const void * W[2]; float * dst[2];      // n_seg = 2: up (-> dst[0]) and gate (-> dst[1]) in one launch
+    int64_t M, K; int n_expert; int64_t estride;                 // the n_expert matrices of W[i] lie estride bytes apart
+    const void * xb; int64_t n_rows;                             // bf16 [n_rows][K], expert-sorted
+    const void * tiles; const int * n_tiles; const int * row_dst; int max_tiles; int nb;
+};
+int b200q_launch_gemm_q_grouped(const b200q_gemm_grouped & g, cudaStream_t st);
+struct b200q_moe_plan_t {
+    int64_t n_rows; int nb; int max_tiles; int64_t estride;
+    size_t off_xb, off_up, off_bounds, off_src, off_dst, off_tiles, off_ntiles, total;     // workspace layout
+};
+// 0: the grouped path covers this type and shape (p filled); -1: type not covered; -2: shape not covered
+int b200q_moe_plan(int type, int64_t m, int64_t k, int n_expert, int n_used, int nb1, int n_tokens, int up_gate, b200q_moe_plan_t * p);
+struct b200q_moe_desc {
+    int type; const void * W; const void * W_gate; int n_expert; const int32_t * ids; const float * x; float * dst;
+    int64_t M, K; int n_used, nb1, n_tokens; int act; float limit;
+};
+int b200q_launch_moe_gemm(const b200q_moe_desc & d, const b200q_moe_plan_t & p, void * ws, cudaStream_t st);

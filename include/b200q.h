@@ -161,9 +161,24 @@ B200Q_API int b200q_add_rows(const float * a, const float * b, float * dst, int6
  * a token, nb1 = n_used: one column per slot); dst f32 [n_tokens][n_used][m]:  dst[t][e] = W[ids[t][e]] . x[t][e % nb1]
  * (W_gate != NULL: unary(W_gate[id] . x) * (W[id] . x)).  Expert ids are resolved on the device.  The quantised activation columns of a launch live
  * in shared memory (200 KB of q8_1): batches whose n_tokens * nb1 columns exceed that are walked in token chunks by the same kernel (functional
- * path for MoE prefill; a grouped tensor-core GEMM over expert-sorted tokens is not built). */
+ * path for MoE prefill when the type or shape has no grouped GEMM, see below). */
 B200Q_API int b200q_mul_mat_id_vec(int type, const void * W, const void * W_gate, int n_expert, const int32_t * ids, const float * x, float * dst,
                          int64_t m, int64_t k, int n_used, int nb1, int n_tokens, int unary, float limit, void * stream);
+/* ---- MoE prefill: the same ops as a grouped tcgen05 GEMM over expert-sorted tokens (ggml_cuda_mul_mat_id with mul_mat_q_id, ggml-cuda.cu:3210-3307).
+ * On the device: route (count the slots per expert, scan, sort the slots by expert, one tile-table entry per 128/256/512-token tile of each
+ * expert), gather the routed activation columns as bf16, one GEMM launch that dequantises the expert weights inside the kernel (up and gate
+ * as two segments of that launch for W_gate != NULL, then the unary-mul).  Nothing is read back to the host: the call can be captured in
+ * a CUDA graph.  No split-K: the result is bit-identical from run to run.  Types: IQ4_NL, Q4_0, Q4_1, Q5_0, Q5_1, Q4_K, Q5_K, IQ4_K,
+ * IQ5_K with k % 256 == 0 and n_expert <= 512 (b200q_mul_mat_id_gemm returns B200Q_E_TYPE / B200Q_E_SHAPE otherwise).
+ * b200q_mul_mat_id_workspace: device bytes the grouped path needs (256-byte aligned workspace), 0 if the type / shape is not covered;
+ * up_gate != 0 for GGML_OP_MOE_FUSED_UP_GATE.  b200q_mul_mat_id: the dispatcher (what the graph nodes call): the grouped GEMM for covered
+ * types and shapes at or above a batch threshold set from measurement (scripts/moe_prefill_bench.py, DESIGN.md §4), b200q_mul_mat_id_vec
+ * otherwise (workspace may then be NULL). */
+B200Q_API size_t b200q_mul_mat_id_workspace(int type, int64_t m, int64_t k, int n_expert, int n_used, int nb1, int n_tokens, int up_gate);
+B200Q_API int b200q_mul_mat_id_gemm(int type, const void * W, const void * W_gate, int n_expert, const int32_t * ids, const float * x, float * dst,
+                          int64_t m, int64_t k, int n_used, int nb1, int n_tokens, int unary, float limit, void * workspace, size_t workspace_bytes, void * stream);
+B200Q_API int b200q_mul_mat_id(int type, const void * W, const void * W_gate, int n_expert, const int32_t * ids, const float * x, float * dst,
+                     int64_t m, int64_t k, int n_used, int nb1, int n_tokens, int unary, float limit, void * workspace, size_t workspace_bytes, void * stream);
 /* same through HOST activations/results: H2D(x) -> mul_mat -> D2H(dst), synchronous (end-to-end entry point) */
 B200Q_API int b200q_mul_mat_host(int type, const void * W_planes_dev, const float * x_host, float * dst_host,
                        int64_t m, int64_t k, int64_t n, void * stream);
